@@ -26,6 +26,12 @@ every ready task is assigned in that one tick and value = tasks / tick time.
   cpu_baseline / --impl reference   the oracle (restated reference tick, HiGHS 1.12.0) on the SAME workload, single-
             threaded like the reference (Rc<RefCell<Core>>), with the reference's solver defaults relaxed to a 1 % MIP gap
             and a 2 s cap (parity.ORACLE_FAST; `solver_hit_cap` says whether the cap was reached).
+
+--dump-outputs DIR writes what the last timed step returned to its caller, so that two builds can be compared output for
+output (the inputs are seeded: the same arguments give the same inputs): the assignment records as assignment_task (float64),
+assignment_worker, assignment_variant, assignment_kind (float32) and the free vectors after the tick as free_after [W][R]
+(float64), one DIR/<name>.npy each; with several GPUs every rank writes its own files (<name>.rank<r>.npy).  Above 64 MB in
+all, a fixed seeded sample of the records is written, with their positions in assignment_row.
 """
 from __future__ import annotations
 
@@ -43,6 +49,7 @@ import traceback
 import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
+sys.dont_write_bytecode = True          # the benchmark leaves the source tree as it found it
 sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(ROOT, "tests"))
 
@@ -58,6 +65,29 @@ CFG5 = {"name": "cfg5-M1", "tasks_per_gpu": 1_250_000, "workers": 1024, "free_sc
                     "Q=16 Zipf(1.1), 8 priorities, one tick, all assignable"}
 BYTES_CONTRACT = 36      # SURVEY.md §8(d): V*R*4 amounts + 8 priority + 4 class/flags read, 8 written per assignment (cfg2, cfg5)
 BYTES_INTERNED = 20      # what the path moves with interned classes: 4 key read (count) + 4 key read (emit) + 8 assignment + 4 key write-back
+DUMP_BYTES = 64 << 20    # --dump-outputs: all files of all ranks together
+DUMP_ROW_BYTES = 28      # one dumped record: task (8) + worker, variant, kind (4 each) + its position when sampled (8)
+
+
+def dump_outputs(out_dir: str, rank: int, world: int, assignments: np.ndarray, free_after: np.ndarray) -> None:
+    """Writes one step's result (assignment records, free vectors after the tick) as float .npy files (exact: handles are
+    u32, the benchmark's amounts stay below 2^53).  More records than this rank's share of DUMP_BYTES: a fixed seeded
+    sample of them, in output order, with their positions."""
+    os.makedirs(out_dir, exist_ok=True)
+    a = assignments
+    arrays = {}
+    rows = (DUMP_BYTES - world * (free_after.size * 8 + 1024)) // (world * DUMP_ROW_BYTES)     # 1 KB: the .npy headers
+    if a.size > rows:
+        idx = np.sort(np.random.default_rng(0).choice(a.size, size=rows, replace=False))
+        a = a[idx]
+        arrays["assignment_row"] = idx.astype(np.float64)
+    arrays["assignment_task"] = a["task"].astype(np.float64)
+    for f in ("worker", "variant", "kind"):
+        arrays[f"assignment_{f}"] = a[f].astype(np.float32)
+    arrays["free_after"] = free_after.astype(np.float64)
+    sfx = f".rank{rank}" if world > 1 else ""
+    for name, arr in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}{sfx}.npy"), arr)
 
 
 def _peaks():
@@ -180,18 +210,14 @@ def run_reference(args) -> None:
     # the CPU arm has no caches to warm beyond the first import: one untimed step on cfg2 (6 s), none on cfg5 (40-100 s each)
     for i in range(min(args.warmup, 1) if cfg["workers"] <= 256 else 0):
         oracle_step(cfg, 100 + i)
+    # every step is the FULL workload (6-20 s of CPU work each on cfg2, more on cfg5)
     n_tot, t_tot, capped, timed = 0, 0.0, 0, 0
-    t_wall0 = time.perf_counter()
     for i in range(args.steps):
         n, dt, cap = oracle_step(cfg, i)
         n_tot += n
         t_tot += dt
         capped += int(cap)
         timed += 1
-        # every step is the FULL workload (6-20 s of CPU work each); the run is bounded by wall-clock instead of by
-        # a smaller sample: steps beyond the budget are not run and `steps_timed` says how many were
-        if time.perf_counter() - t_wall0 > args.ref_budget_s and timed >= (3 if cfg["workers"] <= 256 else 2):
-            break
     value = n_tot / t_tot if t_tot > 0 else 0.0
     desc = {"value": value, "unit": "assignments/s", "cores": 1, "kind": "port",
             "sample": f"the full workload of one GPU per step ({cfg['tasks_per_gpu']} tasks, {cfg['workers']} workers, one M1 tick; the "
@@ -393,12 +419,15 @@ def run_cuda(args) -> dict:
         scheds[i]._check(lib.hqs_tick_fetch(scheds[i]._ctx, n_tasks, L.ptr(tmp_out), C.byref(out_n), None))
     # every step must have assigned every task of the rank
     n_done_local = 0
+    free_last = np.zeros_like(free)
     for i in range(K):
         s = scheds[Wm + i]
-        s._check(lib.hqs_tick_fetch(s._ctx, n_tasks, L.ptr(tmp_out), C.byref(out_n), None))
+        s._check(lib.hqs_tick_fetch(s._ctx, n_tasks, L.ptr(tmp_out), C.byref(out_n), L.ptr(free_last) if i == K - 1 else None))
         n_done_local = int(out_n.value)
         if world == 1:
             assert out_n.value == n_tasks, f"step {i}: {out_n.value} of {n_tasks} tasks assigned"
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, rank, world, tmp_out[:n_done_local], free_last)
 
     if world > 1:
         t = torch.tensor([ms_total], dtype=torch.float64, device=dev)
@@ -496,7 +525,7 @@ def run_cuda(args) -> dict:
     h_cls, h_prio = pin(wl.task_class), pin(prio)
     out = torch.empty(n_tasks * 8, dtype=torch.uint8).pin_memory().numpy().view(L.assignment_dtype)
     free_after = np.zeros_like(free)
-    n_e2e = max(3, min(K, 10))
+    n_e2e = K
 
     def e2e_step():
         # the rank's tasks are one task array (consecutive handles): class ids and priorities cross PCIe, the handles do not
@@ -568,17 +597,21 @@ def run_cuda(args) -> dict:
 def main() -> None:
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=20)
+    ap.add_argument("--steps", type=int, default=20, help="timed steps (the e2e figure times as many)")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="cuda", choices=["cuda", "reference"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
-    ap.add_argument("--ref-budget-s", type=float, default=200.0,
-                    help="--impl reference: wall-clock budget; after it (and at least 3 steps) no further step is started")
     ap.add_argument("--no-extras", action="store_true", help="skip the M2 drains, the class-pool sweep and the seed sweep")
     ap.add_argument("--no-drain", action="store_true", help="alias of --no-extras")
     ap.add_argument("--nccl-exchange", action="store_true",
                     help="N > 1: all-gather the count vectors with NCCL instead of the fused peer-to-peer exchange")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the last timed step's assignments and free vectors as DIR/<name>.npy (CUDA arm)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "cuda":
+        ap.error("--dump-outputs writes the CUDA arm's outputs")
     args.no_extras = args.no_extras or args.no_drain
     args.warmup = max(args.warmup, 3) if args.impl == "cuda" else args.warmup
     rank = int(os.environ.get("RANK", "0"))
